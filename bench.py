@@ -8,12 +8,14 @@ excluded from the timed region and timed separately).  Five windows per step mak
 20-step run ~3 s, long enough that one slow rank shows up in the per-rank record instead of in the noise.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-cuda]
-                    [--height H --width W] [--windows-per-step S] [--no-extras]
+                    [--height H --width W] [--windows-per-step S] [--no-extras] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = device-resident windows/s, `e2e` = the same metric through the module call
 with pinned-host inputs (6 frames H2D per window) and the 3 images test.py writes (outputs 13, 8, 12) copied back D2H
 inside the timed region.  `--impl reference` times the reference's CPU PyTorch path (the unmodified reference when it
-is present on the machine, else the line-cited oracle port) on REAL 1280x720 windows.
+is present on the machine, else the line-cited oracle port) on REAL 1280x720 windows.  `--dump-outputs DIR` also writes
+what the last timed step returned as DIR/*.npy (dump_outputs), so that two builds can be compared output for output on
+the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -97,18 +99,50 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 64_000_000         # --dump-outputs: at most this much is written per run
+
+
+def dump_outputs(out_dir, windows, budget=DUMP_BYTES, seed=0):
+    """Writes the 14 outputs of every window of one step as out_dir/w<window>_out<k>.npy, float32.  Each file gets an
+    equal share of `budget`; an output larger than its share is stored as a 1-D sample of its flattened elements at
+    sorted indices drawn without replacement by numpy's default_rng(seed) -- the same indices for every output of that
+    size, so the files of two runs or two builds compare element for element.  Returns a summary for the JSON line."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {f"w{i}_out{k:02d}": o for i, outs in enumerate(windows) for k, o in enumerate(outs)}
+    share = (budget - 128 * len(arrays)) // (4 * len(arrays))          # elements per file; 128 B of .npy header each
+    picks, total, sampled = {}, 0, 0
+    for name, t in arrays.items():
+        flat = t.detach().reshape(-1)
+        if flat.numel() > share:
+            n = flat.numel()
+            if n not in picks:
+                idx = np.sort(np.random.default_rng(seed).choice(n, size=share, replace=False))
+                picks[n] = torch.from_numpy(idx).to(flat.device)
+            arr = flat[picks[n]].float().cpu().numpy()
+            sampled += 1
+        else:
+            arr = t.detach().float().cpu().numpy()
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, arr)
+        total += os.path.getsize(path)
+    return {"dir": out_dir, "files": len(arrays), "bytes": total, "sampled_files": sampled,
+            "elements_per_sampled_file": share if sampled else None, "sample_seed": seed}
+
+
 # ------------------------------------------------------------------------------------------------ CPU reference
 def _reference_root():
-    """The unmodified reference, when it exists on this machine (the authoring container; never the GPU box)."""
-    for cand in ("/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.isfile(os.path.join(cand, "models", "archs", "RDN.py")):
+    """A checkout of the unmodified reference (laomao0/BIN): BIN_REFERENCE_ROOT, else baseline/_ref, when present."""
+    for cand in (os.environ.get("BIN_REFERENCE_ROOT"), os.path.join(ROOT, "baseline", "_ref")):
+        if cand and os.path.isfile(os.path.join(cand, "models", "archs", "RDN.py")):
             return cand
     return None
 
 
 def cpu_window_runner():
-    """Returns (run(frames) -> outputs, kind): the reference's own bin_stage4_lstm on CPU when /root/reference (or
-    baseline/_ref) is present -- kind "reference" -- else oracle/bin_oracle.py, the line-cited restatement that
+    """Returns (run(frames) -> outputs, kind): the reference's own bin_stage4_lstm on CPU when a checkout of it is
+    found (_reference_root) -- kind "reference" -- else oracle/bin_oracle.py, the line-cited restatement that
     tests/golden pins to the reference's outputs -- kind "port".  Both are fp32 PyTorch CPU (oneDNN) graphs."""
     import torch
     from oracle import bin_oracle as O
@@ -205,6 +239,8 @@ def run_reference(args):
                                        f"(per-window times {[round(t, 2) for t in ts]}); no pixel-count extrapolation"},
             "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "outputs_finite": bool(all(torch.isfinite(o).all() for o in out))}
+    if args.dump_outputs:
+        line["dump_outputs"] = dump_outputs(args.dump_outputs, [out])
     print(json.dumps(line), flush=True)
 
 
@@ -425,14 +461,19 @@ def run_ours(args):
 
     sampler = ClockSampler(local)
     sampler.start()                              # NVML start-up happens here, long before the timed region
+    keep = args.dump_outputs is not None        # the last timed step then holds all S windows' outputs for dump_outputs
     with torch.no_grad():
         outs = None
         for _ in range(args.warmup):
+            held = []
             for w_ in wins_dev:
                 outs = net(*w_)                  # same statement as the timed loop: the previous window's 14 outputs stay alive
                                                  # while the next window allocates its own, so the caching allocator reaches
                                                  # its steady state here (a one-off 220 ms of cudaMalloc fell into the FIRST
                                                  # timed step when the warm-up discarded its outputs: step_ms 365, 144, 144, ...)
+                if keep:
+                    held.append(outs)            # likewise for what the last timed step holds with --dump-outputs
+        del held
         # Settle: a box that has been idle (the reference arm runs on the CPU first) starts at the maximum clock and the
         # power governor then swings below its steady state for a few seconds (seen as a first bench process 6-12 % slower
         # than every later one on the same box, with `e2e` -- measured later in the same process -- FASTER than the
@@ -455,10 +496,13 @@ def run_ours(args):
         sampler.mark_begin()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         marks = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps)]   # one per step boundary, never waited on in the loop
+        last_step = []                           # with --dump-outputs: the S 14-tuples the last timed step returned
         e0.record()
         for i in range(args.steps):
             for w_ in wins_dev:
                 outs = net(*w_)
+                if keep and i == args.steps - 1:
+                    last_step.append(outs)
             marks[i].record()
         e1.record()
         barrier()
@@ -466,6 +510,8 @@ def run_ours(args):
         ms_dev = e0.elapsed_time(e1)
         step_ms = [a.elapsed_time(b) for a, b in zip([e0] + marks[:-1], marks)]
         clocks = sampler.stop()
+        dump = dump_outputs(args.dump_outputs, last_step) if keep and rank == 0 else None
+        del last_step
         # ---- end-to-end: pinned host -> device, forward, 3 result images -> pinned host -----------
         from bin_b200.pipeline import WindowPipeline
         pipe = WindowPipeline(net, dev)
@@ -598,6 +644,8 @@ def run_ours(args):
         }
         if train_ddp is not None:
             line["train_step_ddp"] = train_ddp
+        if dump is not None:
+            line["dump_outputs"] = dump
         line.update(extras)
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -614,7 +662,12 @@ def main():
     ap.add_argument("--width", type=int, default=1280)
     ap.add_argument("--windows-per-step", type=int, default=5)
     ap.add_argument("--no-extras", action="store_true", help="skip roofline / cpu_baseline / eager / train extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference-cuda":
+        ap.error("--dump-outputs is not supported with --impl reference-cuda")
     if args.impl == "reference-cuda":
         run_reference_cuda(args)
     elif args.impl == "reference":

@@ -1,27 +1,15 @@
-"""TEST INFRASTRUCTURE: the reference's caller-side sequence around the hot path, restated so that it can run on the
-GPU box (where /root/reference does not exist) against the drop-in module.
+"""TEST INFRASTRUCTURE: the reference's caller-side sequence around the hot path, restated so that it can run
+against the drop-in module without the reference installed.
 
-Each step cites the reference lines it follows; nothing here is imported by the product package.  When the real
-reference IS importable on the machine that runs the test (`/root/reference` or `baseline/_ref` holding `models/`),
-`reference_root()` returns it and the tests drive the reference's own `bin_model` class instead of this mirror.
+Each step cites the reference lines it follows; nothing here is imported by the product package.
 """
 from __future__ import annotations
 
-import os
 from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
 import torch.nn as nn
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def reference_root() -> Optional[str]:
-    for cand in ("/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.isfile(os.path.join(cand, "models", "bin_model.py")):
-            return cand
-    return None
 
 
 class CallerModel:

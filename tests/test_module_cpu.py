@@ -186,6 +186,51 @@ def test_bench_reference_arm_line_on_cpu():
     assert r1.returncode == 0 and r1.stdout.strip() == ""
 
 
+def test_bench_dump_outputs(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the 14 outputs of the last timed window as float32 .npy, computed from the
+    fixed seeded inputs (checked against the oracle on those inputs); a step larger than the byte budget is written as
+    the same seeded sample of every output, under the budget, identically from run to run."""
+    import json
+    import subprocess
+    import sys
+    import importlib.util
+    import numpy as np
+    out = tmp_path / "dump"
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--height", "48", "--width", "64",
+           "--steps", "1", "--warmup", "0", "--dump-outputs", str(out)]
+    r = subprocess.run(cmd, env=dict(os.environ, RANK="0"), capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    j = json.loads([l for l in r.stdout.strip().split("\n") if l.startswith("{")][0])
+    assert j["dump_outputs"]["files"] == 14 and j["dump_outputs"]["sampled_files"] == 0
+    assert sorted(p.name for p in out.iterdir()) == [f"w0_out{k:02d}.npy" for k in range(14)]
+    ref = O.window_forward(O.synth_frames(6, 1, 48, 64, seed=1234, smooth=True), O.synth_state_dict(0))
+    for k, want in enumerate(ref):
+        got = np.load(out / f"w0_out{k:02d}.npy")
+        assert got.dtype == np.float32 and got.shape == tuple(want.shape)
+        assert np.abs(got - want.numpy()).max() <= 1e-5, k
+
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    n = 3 * 40 * 50
+    step = [[torch.arange(n, dtype=torch.float32).reshape(1, 3, 40, 50) + 10_000 * k for k in range(14)] for _ in range(2)]
+    budget = 100_000
+    a = bench.dump_outputs(str(tmp_path / "a"), step, budget=budget)
+    b = bench.dump_outputs(str(tmp_path / "b"), step, budget=budget)
+    assert a["files"] == b["files"] == 28 and a["sampled_files"] == 28 and a["bytes"] == b["bytes"] <= budget
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) == a["bytes"]
+    idx = None
+    for w in range(2):
+        for k in range(14):
+            x = np.load(tmp_path / "a" / f"w{w}_out{k:02d}.npy")
+            assert np.array_equal(x, np.load(tmp_path / "b" / f"w{w}_out{k:02d}.npy"))
+            assert x.dtype == np.float32 and x.shape == (a["elements_per_sampled_file"],)
+            i = x - 10_000 * k                                  # the values are the sampled flat indices
+            idx = i if idx is None else idx
+            assert np.array_equal(i, idx)
+    assert np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < n
+
+
 def test_bench_clock_sampler_uses_only_samples_of_the_timed_region():
     """bench.py's ClockSampler: median / min SM clock and throttle reasons come from the samples that arrived between
     mark_begin and mark_end (the sampler itself starts before the warm-up); without nvidia-smi it says so."""

@@ -13,6 +13,8 @@ BIN_MAX_FRAMES = 5
 BIN_BACKBONE_NCONV = 66
 EPI_P8, EPI_PIXSHUF, EPI_FINAL = 0, 1, 2
 ABI_VERSION = 2
+BIN_MAX_METRIC_PAIRS = 64
+SSIM_BOX7, SSIM_GAUSS11 = 0, 1
 
 
 class Act(C.Structure):
@@ -96,6 +98,9 @@ _SIGS = {
                                    C.POINTER(Act), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "bin_adam_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int] + [C.c_float] * 8 + [C.c_void_p]),
     "bin_blur_average_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "bin_image_metrics_workspace_bytes": (C.c_size_t, [C.c_int] * 5),
+    "bin_image_metrics_u8": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)] + [C.c_int] * 5 +
+                             [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
 }
 # measurement tooling (libbin_b200_tools.so, csrc/tools_abi.h) -- bound only when BIN_B200_LIB points at that library
 _TOOLS_SIGS = {

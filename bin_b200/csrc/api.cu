@@ -96,6 +96,9 @@ int launch_u8_to_frame(const uint8_t* img, int h, int w, int pl, int pr, int pt,
 int launch_convlstm_bwd(const float* x, const float* c_prev, const float* h_prev, const float* w, const float* b,
                         const float* dh, const float* dc, float* dgates_ws, float* dx, float* dc_prev, float* dh_prev,
                         float* dw, float* db, int B, int H, int W, cudaStream_t s);
+size_t image_metrics_workspace_bytes(int npairs, int h, int w, int c, int kind);   // metrics.cu
+int launch_image_metrics_u8(const uint8_t* const* a, const uint8_t* const* b, int npairs, int h, int w, int c, int kind,
+                            double* res, void* ws, size_t ws_bytes, cudaStream_t s);
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -842,6 +845,14 @@ int bin_blur_average_u8(const uint8_t* frames, int T, size_t frame_bytes, int wi
                         int nwin, uint8_t* out, bin_stream_t s) {
   if (!frames || !out) return fail(BIN_ERR_ARG, "blur_average: null argument");
   return launch_blur_average_u8(frames, T, frame_bytes, window_size, first_mid, stride, nwin, out, (cudaStream_t)s);
+}
+size_t bin_image_metrics_workspace_bytes(int npairs, int h, int w, int c, int kind) {
+  return image_metrics_workspace_bytes(npairs, h, w, c, kind);
+}
+int bin_image_metrics_u8(const uint8_t* const* a_host, const uint8_t* const* b_host, int npairs, int h, int w, int c,
+                         int kind, double* res, void* ws, size_t ws_bytes, bin_stream_t s) {
+  if (!a_host || !b_host || !res || !ws) return fail(BIN_ERR_ARG, "image_metrics: null argument");
+  return launch_image_metrics_u8(a_host, b_host, npairs, h, w, c, kind, res, ws, ws_bytes, (cudaStream_t)s);
 }
 
 }  // extern "C"

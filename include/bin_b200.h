@@ -256,6 +256,26 @@ int bin_adam_step(const bin_adam_tensor_t* table_dev, const int* chunk_prefix_de
 int bin_blur_average_u8(const uint8_t* frames, int T, size_t frame_bytes, int window_size, int first_mid, int stride,
                         int nwin, uint8_t* out, bin_stream_t s);
 
+/* ---- evaluation metrics (DESIGN 5c rank 5): the PSNR / SSIM / interpolation error of test.py:404-458 and the
+ * validation metrics of bin_model.compute_current_psnr_ssim (bin_model.py:564-589) ------------------------------ */
+/* kind selects the SSIM definition; both are valid-region filters (no border handling):
+ *   BIN_SSIM_BOX7    skimage 0.14-0.16 compare_ssim(X, Y, multichannel=True) with the defaults test.py:35 uses:
+ *                    7x7 uniform window, sample covariance (x49/48), K1 = 0.01, K2 = 0.03, L = 255, map cropped by
+ *                    3 px per side, mean over channels of the per-channel means;
+ *   BIN_SSIM_GAUSS11 utils/util.py:211-231 ssim (and calculate_ssim, :234-252): 11x11 window = outer product of
+ *                    cv2.getGaussianKernel(11, 1.5), population moments, same K1 / K2, [5:-5, 5:-5] crop, mean over
+ *                    every element. */
+enum { BIN_SSIM_BOX7 = 0, BIN_SSIM_GAUSS11 = 1 };
+#define BIN_MAX_METRIC_PAIRS 64
+/* Workspace of one call: per-CTA partial sums (0 for arguments the call would reject). */
+size_t bin_image_metrics_workspace_bytes(int npairs, int h, int w, int c, int kind);
+/* res (device double[npairs][3]) = {mse, mae, ssim} per pair; a_host/b_host: npairs device pointers to h*w*c uint8
+ * (HWC, c = 1 or 3, h and w at least the window size).  mse = mean (a-b)^2 (util.py:203-205; PSNR =
+ * 10 log10(255^2 / mse)), mae = mean |a-b| (test.py:431-435 interpolation error).  Sums are exact integers; the
+ * reduction is deterministic (fixed order, no atomics) and a pair's result does not depend on the other pairs. */
+int bin_image_metrics_u8(const uint8_t* const* a_host, const uint8_t* const* b_host, int npairs, int h, int w, int c,
+                         int kind, double* res, void* ws, size_t ws_bytes, bin_stream_t s);
+
 #ifdef __cplusplus
 }
 #endif

@@ -15,6 +15,8 @@ EPI_P8, EPI_PIXSHUF, EPI_FINAL = 0, 1, 2
 ABI_VERSION = 2
 BIN_MAX_METRIC_PAIRS = 64
 SSIM_BOX7, SSIM_GAUSS11 = 0, 1
+BIN_TRAIN_FRAMES = 17
+BIN_MAX_TRAIN_SAMPLES = 64
 
 
 class Act(C.Structure):
@@ -40,6 +42,10 @@ class ConvArgs(C.Structure):
 
 class Net(C.Structure):
     _fields_ = [("blob", C.c_void_p * 4), ("lstm_w", C.c_void_p * 6), ("lstm_b", C.c_void_p * 6)]
+
+
+class TrainSample(C.Structure):
+    _fields_ = [("src", C.c_void_p * BIN_TRAIN_FRAMES), ("y0", C.c_int), ("x0", C.c_int), ("flip", C.c_int)]
 
 
 class BinB200Error(RuntimeError):
@@ -101,6 +107,7 @@ _SIGS = {
     "bin_image_metrics_workspace_bytes": (C.c_size_t, [C.c_int] * 5),
     "bin_image_metrics_u8": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)] + [C.c_int] * 5 +
                              [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "bin_train_batch_u8": (C.c_int, [C.POINTER(TrainSample)] + [C.c_int] * 5 + [C.c_void_p] * 4),
 }
 # measurement tooling (libbin_b200_tools.so, csrc/tools_abi.h) -- bound only when BIN_B200_LIB points at that library
 _TOOLS_SIGS = {

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbin_b200.so")
-SOURCES = ["conv_igemm.cu", "rdb_tail.cu", "aux_kernels.cu", "wgrad.cu", "metrics.cu", "api.cu"]
+SOURCES = ["conv_igemm.cu", "rdb_tail.cu", "aux_kernels.cu", "wgrad.cu", "metrics.cu", "train_data.cu", "api.cu"]
 HEADERS = ["common.cuh", "internal.h", os.path.join("..", "..", "include", "bin_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]

@@ -99,6 +99,8 @@ int launch_convlstm_bwd(const float* x, const float* c_prev, const float* h_prev
 size_t image_metrics_workspace_bytes(int npairs, int h, int w, int c, int kind);   // metrics.cu
 int launch_image_metrics_u8(const uint8_t* const* a, const uint8_t* const* b, int npairs, int h, int w, int c, int kind,
                             double* res, void* ws, size_t ws_bytes, cudaStream_t s);
+int launch_train_batch_u8(const bin_train_sample_t* samples, int B, int H, int W, int h, int w, float* lqs, float* gtenh,
+                          float* gtinp, cudaStream_t s);   // train_data.cu
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -853,6 +855,11 @@ int bin_image_metrics_u8(const uint8_t* const* a_host, const uint8_t* const* b_h
                          int kind, double* res, void* ws, size_t ws_bytes, bin_stream_t s) {
   if (!a_host || !b_host || !res || !ws) return fail(BIN_ERR_ARG, "image_metrics: null argument");
   return launch_image_metrics_u8(a_host, b_host, npairs, h, w, c, kind, res, ws, ws_bytes, (cudaStream_t)s);
+}
+int bin_train_batch_u8(const bin_train_sample_t* samples, int B, int H, int W, int h, int w, float* lqs, float* gtenh,
+                       float* gtinp, bin_stream_t s) {
+  if (!samples || !lqs || !gtenh || !gtinp) return fail(BIN_ERR_ARG, "train_batch: null argument");
+  return launch_train_batch_u8(samples, B, H, W, h, w, lqs, gtenh, gtinp, (cudaStream_t)s);
 }
 
 }  // extern "C"

@@ -276,6 +276,22 @@ size_t bin_image_metrics_workspace_bytes(int npairs, int h, int w, int c, int ki
 int bin_image_metrics_u8(const uint8_t* const* a_host, const uint8_t* const* b_host, int npairs, int h, int w, int c,
                          int kind, double* res, void* ws, size_t ws_bytes, bin_stream_t s);
 
+/* ---- training batches (DESIGN 5c rank 6): BINDataset.__getitem__ + DataLoader collation, data/BIN_dataset.py:30-183 -- */
+/* One sample: its 17 source frames in output-slot order -- blurry B1..B11 (LQs), sharp I1..I11 (GTenh), sharp
+ * I2..I10 (GTinp); the reference's random reversal (:68-109) is the caller's choice of this order -- and its crop
+ * (rows y0.., columns x0..) and np.fliplr (:155-177).  Each src: device uint8 (H, W, 3) BGR, row-major HWC. */
+#define BIN_TRAIN_FRAMES 17
+#define BIN_MAX_TRAIN_SAMPLES 64 /* samples per kernel launch (the table travels in the kernel parameters) */
+typedef struct {
+  const uint8_t* src[BIN_TRAIN_FRAMES];
+  int y0, x0, flip;
+} bin_train_sample_t;
+/* samples: host array of B >= 1 entries (one launch per BIN_MAX_TRAIN_SAMPLES of them; no copy, no synchronisation).
+ * Writes fp32 float32(u8)/255 RGB crops of h x w (1 <= h <= H, 1 <= w <= W, crop inside the frame) slot-major:
+ * lqs [6][B][3][h][w], gtenh [6][B][3][h][w], gtinp [5][B][3][h][w]. */
+int bin_train_batch_u8(const bin_train_sample_t* samples, int B, int H, int W, int h, int w, float* lqs, float* gtenh,
+                       float* gtinp, bin_stream_t s);
+
 #ifdef __cplusplus
 }
 #endif
